@@ -365,6 +365,9 @@ def bench_b200(args, rank, world):
     resident_steps(args.steps, open_timed_region)
     torch.cuda.synchronize()
     t_res = max_over_ranks(time.perf_counter() - clock["t0"])
+    # what the last timed step handed its callers: one JPEG/R stream per frame
+    # (rank 0's frames only: the dump stays within its size budget whatever the number of ranks)
+    last_streams = [stream_bytes(lib, hnd.h) for hnd in handles] if args.dump_outputs and rank == 0 else None
     l0 = clock["l0"]
     launches = lib.uhdr_b200_kernel_launches() - l0
     lib.uhdr_b200_set_kernel_timing(1)
@@ -439,6 +442,9 @@ def bench_b200(args, rank, world):
     torch.cuda.synchronize()
     t_dec = max_over_ranks(time.perf_counter() - t0)
     dec_value = world * dec_handles * dec_per * (W8K * H8K / 1e6) / t_dec
+    if last_streams is not None:
+        dump_outputs(args.dump_outputs, last_streams, lib.uhdr_get_decoded_image(decs[0]).contents)
+        del last_streams
     for d in decs:
         lib.uhdr_release_decoder(d)
 
@@ -586,6 +592,41 @@ def bench_b200(args, rank, world):
     emit(line)
     if world > 1:
         dist.destroy_process_group()
+
+
+def stream_bytes(lib, handle):
+    o = lib.uhdr_get_encoded_stream(handle).contents
+    return C.string_at(o.data, o.data_sz)
+
+
+def dump_outputs(out_dir, streams, decoded):
+    """--dump-outputs: what the timed paths returned in their last step on rank 0, as .npy files (float32 /
+    float64) that two builds can be compared with, at most 48 MB in all:
+      stream_length.npy         float64 (F,)       bytes of each frame's JPEG/R file (API-1 encode arm)
+      stream_bytes_sample.npy   float32 (F, S)     byte values, S = min(2^18, 2^23 / F): the first min(4096, S)
+                                                   bytes of each file (headers, metadata), then offsets drawn
+                                                   uniformly from the rest with numpy RandomState(frame index),
+                                                   in increasing order
+      decode_8k_rgba_sample.npy float32 (2^20, 4)  RGBA half-float pixels of the 8K decode arm, at 2^20 pixel
+                                                   indices drawn with RandomState(0), in increasing order"""
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(streams)
+    per = max(1, min(1 << 18, (32 << 20) // 4 // max(1, n)))
+    head = min(4096, per)
+    sample = np.zeros((n, per), np.float32)
+    for i, s in enumerate(streams):
+        b = np.frombuffer(s, np.uint8)
+        k = min(head, b.size)
+        rest = np.sort(np.random.RandomState(i).randint(k, max(k + 1, b.size), per - k)) if b.size > k else np.zeros(per - k, np.int64)
+        idx = np.concatenate([np.arange(k), rest]) if b.size else np.zeros(per, np.int64)
+        sample[i] = b[idx] if b.size else 0
+    np.save(os.path.join(out_dir, "stream_length.npy"), np.array([len(s) for s in streams], np.float64))
+    np.save(os.path.join(out_dir, "stream_bytes_sample.npy"), sample)
+    w, h = decoded.w, decoded.h
+    px = np.ctypeslib.as_array(C.cast(decoded.planes[0], C.POINTER(C.c_uint16)), (h, decoded.stride[0] * 4))[:, :w * 4]
+    flat = px.reshape(h * w, 4)
+    pick = np.sort(np.random.RandomState(0).randint(0, h * w, 1 << 20))
+    np.save(os.path.join(out_dir, "decode_8k_rgba_sample.npy"), flat[pick].view(np.float16).astype(np.float32))
 
 
 def apply_8k(lib, hbm, iters=6):
@@ -925,6 +966,8 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--frames", type=int, default=32, help="4K frames per GPU per step (config 4: 32 per GPU)")
     ap.add_argument("--slots", type=int, default=8, help="concurrent encoder handles (host threads) per GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what they returned in the last step to DIR/*.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))

@@ -46,10 +46,11 @@ def test_surface_compiles_and_links_against_include(tmp_path):
 
 @pytest.mark.gpu
 def test_surface_behaves_like_the_reference(gpu, tmp_path):
-    d = os.path.join(T.ROOT, "oracle", "_ref", "fixtures")
-    p, y = os.path.join(d, "raw_p010_image.p010"), os.path.join(d, "raw_yuv420_image.yuv420")
-    if not (os.path.exists(p) and os.path.exists(y)):
-        pytest.skip("720p fixtures not present")
+    # the reference's 1280x720 fixtures (stored compressed in tests/golden), as the files the program reads
+    pb, yb = T.load_fixture_720p()
+    p, y = str(tmp_path / "raw_p010_image.p010"), str(tmp_path / "raw_yuv420_image.yuv420")
+    pb.tofile(p)
+    yb.tofile(y)
     exe = _build(tmp_path)
     r = subprocess.run([exe, p, y], capture_output=True, text=True, timeout=300)
     assert r.returncode == 0, (r.stdout[-2000:], r.stderr[-2000:])

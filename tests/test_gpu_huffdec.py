@@ -91,14 +91,12 @@ def test_device_entropy_decoder_whole_file(gpu, oracle_libs):
 def test_device_entropy_decoder_4k_against_reference(gpu, oracle_libs):
     """config 4 geometry: a 3840x2160 file (≈50k subsequences per scan, both scans decoded concurrently on
     two streams) -> pixels, gain map and metadata identical to the reference decoder's."""
-    if not oracle_libs.have_ref():
-        pytest.skip("reference build not available")
     import bench
     w, h = 3840, 2160
     p, y = bench.make_frame(w, h, 3)
     hdr, sdr, keep = bench.frame_descs(p, y, w, h)
     mine = T.UhdrApi(gpu.lib)
-    ref = T.UhdrApi(oracle_libs.Ref().lib)
+    ref = T.UhdrApi(oracle_libs.Ref().lib) if oracle_libs.have_ref() else None
     data = mine.encode(hdr, sdr)
     lib = gpu.lib
     lib.uhdr_b200_entropy_decoder_stats.restype = None
@@ -106,10 +104,9 @@ def test_device_entropy_decoder_4k_against_reference(gpu, oracle_libs):
     pa, ga, ma, cga = mine.decode(data)
     s1 = _stats(lib)
     assert s1[0] == s0[0] + 2 and s1[1] == s0[1], (s0, s1)
-    pb, gb, mb, cgb = ref.decode(data)
-    assert T.md_equal(ma, mb) and cga == cgb
-    assert (ga == gb).all()
-    assert (pa == pb).all(), int((pa != pb).sum())
+    # recorded results describe the reference's decode of the reference's own file: the stream must be that file
+    assert T.same(data, T.from_reference("huffdec/4k_file", lambda: ref.encode(hdr, sdr)))
+    assert T.same((pa, ga, ma, cga), T.from_reference("huffdec/4k_decoded", lambda: ref.decode(data)))
 
 
 def test_corrupted_scans_agree_with_host_decoder(gpu, oracle_libs):

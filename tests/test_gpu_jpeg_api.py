@@ -1,6 +1,7 @@
 """GPU parity of the JPEG block stage and of the drop-in C API (uhdr_encode / uhdr_decode): the
 coefficient blocks and the complete byte streams must equal the CPU checker's, and whole files must
-be byte-identical to what the reference's own uhdr_encode writes."""
+be byte-identical to what the reference's own uhdr_encode writes (the reference build where oracle/_ref is
+present, else the digests recorded from it, tests/golden/reference_digests.json)."""
 import ctypes as C
 
 import numpy as np
@@ -100,6 +101,16 @@ def test_decode_planes(gpu, oracle_libs):
                     assert tuple(got[yy, xx]) == (r[0], g[0], b[0], 255)
 
 
+def _ref_api(oracle_libs):
+    """the reference's C API, or None where its build is absent (recorded results stand in)"""
+    return T.UhdrApi(oracle_libs.Ref().lib) if oracle_libs.have_ref() else None
+
+
+def _ref_encoded(key, ref, mine, hdr, sdr, **opts):
+    """a JPEG/R the reference wrote: live, or the product's file checked against the reference's digest"""
+    return T.reference_file(key, lambda: ref.encode(hdr, sdr, **opts), mine=lambda: mine.encode(hdr, sdr, **opts))
+
+
 def _frames(w, h, kind="smooth"):
     hb = T.make_p010(w, h, kind)
     sb = T.make_yuv420(w, h, kind)
@@ -112,46 +123,38 @@ def _frames(w, h, kind="smooth"):
 @pytest.mark.parametrize("opts", [{}, {"scale": 4, "multichannel": 0}, {"preset": A.USAGE_REALTIME, "quality": 80}])
 def test_uhdr_encode_api1_file_bytes(gpu, oracle_libs, w, h, kind, opts):
     """uhdr_encode (API-1) through the drop-in C ABI == the reference's uhdr_encode, byte for byte."""
-    if not oracle_libs.have_ref():
-        pytest.skip("reference build not available")
-    ref = T.UhdrApi(oracle_libs.Ref().lib)
+    ref = _ref_api(oracle_libs)
     mine = T.UhdrApi(gpu.lib)
     hdr, sdr, keep = _frames(w, h, kind)
     a = mine.encode(hdr, sdr, **opts)
-    b = ref.encode(hdr, sdr, **opts)
-    assert len(a) == len(b), (len(a), len(b))
-    assert a == b
+    b = T.from_reference("jpeg_api/api1/%dx%d/%s/%s" % (w, h, kind, sorted(opts.items())), lambda: ref.encode(hdr, sdr, **opts))
+    assert T.same(a, b), (len(a), b if isinstance(b, T.Recorded) else len(b))
 
 
 def test_uhdr_decode_pixels(gpu, oracle_libs):
     """uhdr_decode of a reference-encoded file: RGBA half-float pixels, decoded gain map and metadata
     identical to the reference decoder's."""
-    if not oracle_libs.have_ref():
-        pytest.skip("reference build not available")
-    ref = T.UhdrApi(oracle_libs.Ref().lib)
+    ref = _ref_api(oracle_libs)
     mine = T.UhdrApi(gpu.lib)
     for (w, h, opts) in ((640, 368, {}), (640, 368, {"scale": 4, "multichannel": 0}), (1280, 720, {"scale": 2})):
         hdr, sdr, keep = _frames(w, h)
-        data = ref.encode(hdr, sdr, **opts)
+        key = "jpeg_api/decode/%dx%d/%s" % (w, h, sorted(opts.items()))
+        data = _ref_encoded(key + "/file", ref, mine, hdr, sdr, **opts)
         for fmt, ct in ((A.FMT_RGBAF16, A.CT_LINEAR), (A.FMT_RGBA1010102, A.CT_PQ)):
-            pa, ga, ma, cga = mine.decode(data, fmt, ct)
-            pb, gb, mb, cgb = ref.decode(data, fmt, ct)
-            assert T.md_equal(ma, mb)
-            assert (ga == gb).all()
-            assert cga == cgb
-            assert (pa == pb).all(), (w, h, opts, fmt, int((pa != pb).sum()))
+            got = mine.decode(data, fmt, ct)   # pixels, gain map, metadata, gamut
+            want = T.from_reference(key + "/fmt%d_ct%d" % (fmt, ct), lambda: ref.decode(data, fmt, ct))
+            assert T.same(got, want), (w, h, opts, fmt)
 
 
 @pytest.mark.parametrize("w,h,kind", [(640, 368, "smooth"), (1280, 720, "noise")])
 def test_uhdr_encode_api0_file_bytes(gpu, oracle_libs, w, h, kind):
     """API-0 (toneMap + one-pass gain map + both JPEGs) == the reference's file, byte for byte."""
-    if not oracle_libs.have_ref():
-        pytest.skip("reference build not available")
-    ref = T.UhdrApi(oracle_libs.Ref().lib)
+    ref = _ref_api(oracle_libs)
     mine = T.UhdrApi(gpu.lib)
     hdr, sdr, keep = _frames(w, h, kind)
     for opts in ({}, {"multichannel": 0}, {"scale": 2}):
-        assert mine.encode(hdr, None, **opts) == ref.encode(hdr, None, **opts), opts
+        want = T.from_reference("jpeg_api/api0/%dx%d/%s/%s" % (w, h, kind, sorted(opts.items())), lambda: ref.encode(hdr, None, **opts))
+        assert T.same(mine.encode(hdr, None, **opts), want), opts
 
 
 def _rgba_frames(w, h, hdr_kind):
@@ -171,17 +174,17 @@ def _rgba_frames(w, h, hdr_kind):
 def test_uhdr_encode_packed_intents_file_bytes(gpu, oracle_libs, hdr_kind):
     """RGBA1010102 / RGBA half-float HDR intents and the RGBA8888 SDR intent (convert_raw_input_to_ycbcr,
     4:4:4 base image): API-0 and API-1 files equal the reference's byte for byte."""
-    if not oracle_libs.have_ref():
-        pytest.skip("reference build not available")
-    ref = T.UhdrApi(oracle_libs.Ref().lib)
+    ref = _ref_api(oracle_libs)
     mine = T.UhdrApi(gpu.lib)
     for (w, h) in ((320, 192), (648, 364)):
         hdr, sdr, keep = _rgba_frames(w, h, hdr_kind)
-        a, b = mine.encode(hdr, None), ref.encode(hdr, None)
-        assert a == b, ("api0", hdr_kind, w, h, len(a), len(b))
+        key = "jpeg_api/packed/%s/%dx%d" % (hdr_kind, w, h)
+        a, b = mine.encode(hdr, None), T.from_reference(key + "/api0", lambda: ref.encode(hdr, None))
+        assert T.same(a, b), ("api0", hdr_kind, w, h, len(a))
         for opts in ({}, {"scale": 2, "multichannel": 0}):
-            a, b = mine.encode(hdr, sdr, **opts), ref.encode(hdr, sdr, **opts)
-            assert a == b, ("api1", hdr_kind, w, h, opts, len(a), len(b))
+            a = mine.encode(hdr, sdr, **opts)
+            b = T.from_reference(key + "/api1/%s" % sorted(opts.items()), lambda: ref.encode(hdr, sdr, **opts))
+            assert T.same(a, b), ("api1", hdr_kind, w, h, opts, len(a))
 
 
 @pytest.mark.parametrize("subsampling", [2, 1, 0])
@@ -220,35 +223,30 @@ def test_decode_rgb_of_subsampled_streams(gpu, oracle_libs, subsampling):
 def test_uhdr_decode_sdr_output(gpu, oracle_libs):
     """uhdr_decode with UHDR_CT_SRGB / RGBA8888: the base image through libjpeg's RGB path, gain map and
     metadata still available -- identical to the reference decoder."""
-    if not oracle_libs.have_ref():
-        pytest.skip("reference build not available")
-    ref = T.UhdrApi(oracle_libs.Ref().lib)
+    ref = _ref_api(oracle_libs)
     mine = T.UhdrApi(gpu.lib)
     for (w, h, opts) in ((640, 368, {}), (322, 182, {"scale": 2, "multichannel": 0})):
         hdr, sdr, keep = _frames(w, h)
-        data = ref.encode(hdr, sdr, **opts)
-        pa, ga, ma, cga = mine.decode(data, A.FMT_RGBA8888, A.CT_SRGB)
-        pb, gb, mb, cgb = ref.decode(data, A.FMT_RGBA8888, A.CT_SRGB)
-        assert T.md_equal(ma, mb) and cga == cgb
-        assert (ga == gb).all()
-        assert (pa == pb).all(), (w, h, opts, int((pa != pb).sum()))
+        key = "jpeg_api/decode_sdr/%dx%d/%s" % (w, h, sorted(opts.items()))
+        data = _ref_encoded(key + "/file", ref, mine, hdr, sdr, **opts)
+        got = mine.decode(data, A.FMT_RGBA8888, A.CT_SRGB)
+        want = T.from_reference(key + "/decoded", lambda: ref.decode(data, A.FMT_RGBA8888, A.CT_SRGB))
+        assert T.same(got, want), (w, h, opts)
 
 
 def test_uhdr_decode_444_base(gpu, oracle_libs):
     """files written from an RGBA8888 SDR intent carry a 4:4:4 base image: decode (half float, PQ
     1010102 and SDR outputs) == the reference decoder."""
-    if not oracle_libs.have_ref():
-        pytest.skip("reference build not available")
-    ref = T.UhdrApi(oracle_libs.Ref().lib)
+    ref = _ref_api(oracle_libs)
     mine = T.UhdrApi(gpu.lib)
     hdr, sdr, keep = _rgba_frames(328, 200, "pq")
     for opts in ({}, {"scale": 2}):
-        data = ref.encode(hdr, sdr, **opts)
+        key = "jpeg_api/decode_444/328x200/%s" % sorted(opts.items())
+        data = _ref_encoded(key + "/file", ref, mine, hdr, sdr, **opts)
         for fmt, ct in ((A.FMT_RGBAF16, A.CT_LINEAR), (A.FMT_RGBA1010102, A.CT_PQ), (A.FMT_RGBA1010102, A.CT_HLG), (A.FMT_RGBA8888, A.CT_SRGB)):
-            pa, ga, ma, cga = mine.decode(data, fmt, ct)
-            pb, gb, mb, cgb = ref.decode(data, fmt, ct)
-            assert T.md_equal(ma, mb) and cga == cgb and (ga == gb).all()
-            assert (pa == pb).all(), (opts, fmt, ct, int((pa != pb).sum()))
+            got = mine.decode(data, fmt, ct)
+            want = T.from_reference(key + "/fmt%d_ct%d" % (fmt, ct), lambda: ref.decode(data, fmt, ct))
+            assert T.same(got, want), (opts, fmt, ct)
 
 
 def test_encode_batch_matches_single_encodes(gpu, oracle_libs):
@@ -286,16 +284,16 @@ def test_encode_batch_matches_single_encodes(gpu, oracle_libs):
 def test_uhdr_encode_api2_api3_file_bytes(gpu, oracle_libs, w, h, kind):
     """Encode API-2 (raw hdr + raw sdr + compressed sdr) and API-3 (raw hdr + compressed sdr: the JPEG is
     decoded on the device, the gain map computed against it with BT.601 luma): files equal the reference's."""
-    if not oracle_libs.have_ref():
-        pytest.skip("reference build not available")
     PIL = pytest.importorskip("PIL.Image")
     import io
-    ref = T.UhdrApi(oracle_libs.Ref().lib)
+    ref = _ref_api(oracle_libs)
     mine = T.UhdrApi(gpu.lib)
     hdr, sdr, keep = _frames(w, h, kind)
     # compressed sdr intents: the reference's own base image (4:2:0, with ICC) and a Pillow file (4:2:0 / 4:4:4, no ICC)
     from test_probe_cpu import _probe
-    base_ref = _probe(oracle_libs.Ref().lib, ref.encode(hdr, sdr))["base_image"]
+    key = "jpeg_api/api2_api3/%dx%d/%s" % (w, h, kind)
+    base_ref = T.reference_file(key + "/base_image", lambda: _probe(ref.lib, ref.encode(hdr, sdr))["base_image"],
+                                mine=lambda: _probe(gpu.lib, mine.encode(hdr, sdr))["base_image"])
     rgb = np.random.RandomState(5).randint(0, 256, (h, w, 3)).astype(np.uint8)
     pil = {}
     for ss in (2, 0):
@@ -307,8 +305,7 @@ def test_uhdr_encode_api2_api3_file_bytes(gpu, oracle_libs, w, h, kind):
              ("api3", pil[2], None, A.CG_P3, {}), ("api3", pil[0], None, A.CG_BT709, {"scale": 2}),
              ("api3", pil[2], None, -1, {}),           # no ICC and no gamut: error in both
              ("api3", base_ref, None, A.CG_BT2100, {})]  # configured gamut contradicts the ICC: error in both
-    for name, jpg, raw, cg, opts in cases:
-        a = mine.encode_with_compressed_sdr(hdr, jpg, raw, cg, **opts)
-        b = ref.encode_with_compressed_sdr(hdr, jpg, raw, cg, **opts)
-        assert type(a) is type(b), (name, cg, opts, a if isinstance(a, int) else len(a), b if isinstance(b, int) else len(b))
-        assert a == b, (name, cg, opts)
+    for i, (name, jpg, raw, cg, opts) in enumerate(cases):
+        a = mine.encode_with_compressed_sdr(hdr, jpg, raw, cg, **opts)   # the file, or the error code
+        b = T.from_reference(key + "/case%d" % i, lambda: ref.encode_with_compressed_sdr(hdr, jpg, raw, cg, **opts))
+        assert T.same(a, b), (name, cg, opts, a if isinstance(a, int) else len(a))

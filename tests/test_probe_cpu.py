@@ -38,16 +38,32 @@ def _probe(lib, data):
         lib.uhdr_release_decoder(dec)
 
 
+def _summary(p):
+    """what a caller of uhdr_dec_probe gets: the verdict, or dimensions, metadata and the four blocks"""
+    if "error" in p:
+        return ("error", p["error"])
+    return (p["dims"], p["md"], p["exif"], p["icc"], p["base_image"], p["gainmap_image"])
+
+
+def _ref_lib(oracle_libs):
+    """the reference build, or None where it is absent (recorded results stand in)"""
+    return oracle_libs.Ref().lib if oracle_libs.have_ref() else None
+
+
+def _seed_file(oracle_libs, w=64, h=64):
+    """a JPEG/R the reference encoder wrote from the smooth test frames"""
+    hb = T.make_p010(w, h, "smooth")
+    sb = T.make_yuv420(w, h, "smooth")
+    hdr, k1 = A.p010_image(hb, w, h, A.CG_BT2100, A.CT_HLG, A.CR_LIMITED)
+    sdr, k2 = A.yuv420_image(sb, w, h, A.CG_BT709)
+    return T.reference_file("probe/file_%dx%d" % (w, h), lambda: T.UhdrApi(oracle_libs.Ref().lib).encode(hdr, sdr))
+
+
 @pytest.mark.parametrize("opts", [{}, {"scale": 4, "multichannel": 0}, {"preset": A.USAGE_REALTIME, "quality": 60}, {"api0": True}])
 def test_probe_matches_reference(oracle_libs, opts):
-    if not oracle_libs.have_ref():
-        pytest.skip("reference build not available")
-    ref_lib = oracle_libs.Ref().lib
-    mine_lib = C.CDLL(oracle_libs.B200_SO) if hasattr(oracle_libs, "B200_SO") else None
-    if mine_lib is None:
-        import os
-        mine_lib = C.CDLL(os.path.join(oracle_libs.ROOT, "libultrahdr_b200", "libuhdr_b200.so"))
-    ref = T.UhdrApi(ref_lib)
+    import os
+    ref_lib = _ref_lib(oracle_libs)
+    mine_lib = C.CDLL(os.path.join(oracle_libs.ROOT, "libultrahdr_b200", "libuhdr_b200.so"))
     w, h = 320, 192
     hb = T.make_p010(w, h, "smooth")
     sb = T.make_yuv420(w, h, "smooth")
@@ -55,34 +71,26 @@ def test_probe_matches_reference(oracle_libs, opts):
     sdr, k2 = A.yuv420_image(sb, w, h, A.CG_BT709)
     o = dict(opts)
     api0 = o.pop("api0", False)
-    data = ref.encode(hdr, None if api0 else sdr, **o)
-    a, b = _probe(mine_lib, data), _probe(ref_lib, data)
-    assert "error" not in a and "error" not in b, (a, b)
-    assert a["dims"] == b["dims"]
-    assert T.md_equal(a["md"], b["md"])
-    for k in ("exif", "icc", "base_image", "gainmap_image"):
-        assert a[k] == b[k], (k, len(a[k]), len(b[k]))
+    key = "probe/match/%s" % sorted(opts.items())
+    data = T.reference_file(key + "/file", lambda: T.UhdrApi(ref_lib).encode(hdr, None if api0 else sdr, **o))
+    a = _probe(mine_lib, data)
+    assert "error" not in a, a
+    b = T.from_reference(key + "/probe", lambda: _summary(_probe(ref_lib, data)))
+    assert T.same(_summary(a), b)
 
 
 def test_probe_rejects_what_the_reference_rejects(oracle_libs):
-    if not oracle_libs.have_ref():
-        pytest.skip("reference build not available")
     import os
-    ref_lib = oracle_libs.Ref().lib
+    ref_lib = _ref_lib(oracle_libs)
     mine_lib = C.CDLL(os.path.join(oracle_libs.ROOT, "libultrahdr_b200", "libuhdr_b200.so"))
-    ref = T.UhdrApi(ref_lib)
-    w, h = 64, 64
-    hb = T.make_p010(w, h, "smooth")
-    sb = T.make_yuv420(w, h, "smooth")
-    hdr, k1 = A.p010_image(hb, w, h, A.CG_BT2100, A.CT_HLG, A.CR_LIMITED)
-    sdr, k2 = A.yuv420_image(sb, w, h, A.CG_BT709)
-    good = ref.encode(hdr, sdr)
+    good = _seed_file(oracle_libs)
     second = good.index(b"\xff\xd8", 4)
     # inputs the reference build itself handles: compare the verdicts
-    for bad in (good[:second],            # primary image only: no gain map
-                b"\x00" * 64):            # not a JPEG at all
-        a, b = _probe(mine_lib, bad), _probe(ref_lib, bad)
-        assert ("error" in a) == ("error" in b), (len(bad), a.get("error"), b.get("error"))
+    for name, bad in (("primary_only", good[:second]),   # primary image only: no gain map
+                      ("zeros", b"\x00" * 64)):           # not a JPEG at all
+        a = _probe(mine_lib, bad)
+        b = T.from_reference("probe/verdict/" + name, lambda: "error" in _probe(ref_lib, bad))
+        assert T.same("error" in a, b), (name, a.get("error"), b)
     # truncated streams (the reference build used as checker crashes on these): must be refused cleanly
     for bad in (good[:200], good[:second] + good[second:second + 40], good[:3], good[:second + 2]):
         assert "error" in _probe(mine_lib, bad), len(bad)
@@ -91,17 +99,9 @@ def test_probe_rejects_what_the_reference_rejects(oracle_libs):
 def test_probe_survives_mutated_streams(oracle_libs):
     """byte flips, truncations and deletions all over a valid file: the host-side parsers (container
     split, marker walk, ISO 21496-1 metadata, ICC gamut) must answer with a verdict, never crash."""
-    if not oracle_libs.have_ref():
-        pytest.skip("reference build not available (used here only to write the seed file)")
     import os
     mine_lib = C.CDLL(os.path.join(oracle_libs.ROOT, "libultrahdr_b200", "libuhdr_b200.so"))
-    ref = T.UhdrApi(oracle_libs.Ref().lib)
-    w, h = 64, 64
-    hb = T.make_p010(w, h, "smooth")
-    sb = T.make_yuv420(w, h, "smooth")
-    hdr, k1 = A.p010_image(hb, w, h, A.CG_BT2100, A.CT_HLG, A.CR_LIMITED)
-    sdr, k2 = A.yuv420_image(sb, w, h, A.CG_BT709)
-    good = bytearray(ref.encode(hdr, sdr))
+    good = bytearray(_seed_file(oracle_libs))
     n = len(good)
     rs = np.random.RandomState(20240607)
     verdicts = [0, 0]
@@ -129,22 +129,14 @@ def test_probe_survives_mutated_streams(oracle_libs):
 def test_host_parsers_under_sanitizers(oracle_libs, tmp_path):
     """the same mutations, 6000 of them, through the host sources compiled with AddressSanitizer and
     UndefinedBehaviorSanitizer (tests/cpp/host_parsers_fuzz.cpp): no report may appear."""
-    if not oracle_libs.have_ref():
-        pytest.skip("reference build not available (used here only to write the seed file)")
     import os
     import shutil
     import subprocess
     if shutil.which("g++") is None:
         pytest.skip("no g++")
     root = oracle_libs.ROOT
-    ref = T.UhdrApi(oracle_libs.Ref().lib)
-    w, h = 64, 64
-    hb = T.make_p010(w, h, "smooth")
-    sb = T.make_yuv420(w, h, "smooth")
-    hdr, k1 = A.p010_image(hb, w, h, A.CG_BT2100, A.CT_HLG, A.CR_LIMITED)
-    sdr, k2 = A.yuv420_image(sb, w, h, A.CG_BT709)
     seed = tmp_path / "seed.jpg"
-    seed.write_bytes(ref.encode(hdr, sdr))
+    seed.write_bytes(_seed_file(oracle_libs))
     exe = str(tmp_path / "fuzz")
     csrc = os.path.join(root, "libultrahdr_b200", "csrc")
     cmd = ["g++", "-std=c++17", "-O1", "-g", "-fsanitize=address,undefined", "-fno-omit-frame-pointer", "-I", csrc,

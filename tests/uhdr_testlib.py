@@ -26,13 +26,12 @@ REF_TURBO_SO = os.path.join(ROOT, "oracle", "_ref", "libuhdr_ref_turbo.so")
 REF_SO = REF_TURBO_SO if os.path.exists(REF_TURBO_SO) else REF_SHIM_SO
 ORACLE_SO = os.path.join(ROOT, "oracle", "liboracle.so")
 GPU_SO = os.environ.get("UHDR_B200_SO") or os.path.join(ROOT, "libultrahdr_b200", "libuhdr_b200.so")
-REF_DATA = "/root/reference/tests/data"
+GOLDEN = os.path.join(ROOT, "tests", "golden")
 SEED = 20240607
 
 
 def ensure_oracle_built():
-    if not os.path.exists(ORACLE_SO) or (os.path.isdir("/root/reference/lib/src")
-                                          and not (os.path.exists(REF_SHIM_SO) and os.path.exists(REF_TURBO_SO))):
+    if not os.path.exists(ORACLE_SO):
         subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "all"],
                               stdout=subprocess.DEVNULL)
 
@@ -43,6 +42,129 @@ def have_ref():
 
 def ref_is_turbo():
     return REF_SO == REF_TURBO_SO and os.path.exists(REF_TURBO_SO)
+
+
+# ------------------------------------------------------------------------------------------------
+# recorded reference results (tests/golden/reference_digests.json, tests/golden/reference/)
+#
+# A parity test asks the reference build for its answer through from_reference() / reference_file().
+# Where oracle/_ref is built, the reference computes it; everywhere else the SHA-256 recorded from an
+# earlier run of the reference stands in, so the comparison is made on every machine.  Recording:
+#     UHDR_RECORD_REFERENCE=<dir> python -m pytest tests      (with oracle/_ref built)
+# writes <dir>/reference_digests.json and <dir>/reference/*.bin; copy them into tests/golden/.
+# ------------------------------------------------------------------------------------------------
+REF_DIGESTS = os.path.join(GOLDEN, "reference_digests.json")
+REF_BLOBS = os.path.join(GOLDEN, "reference")
+_digests_cache = None
+
+
+def digest(x):
+    """SHA-256 over a canonical form of bytes, arrays, strings, ctypes structures, ints and tuples of them"""
+    import hashlib
+    h = hashlib.sha256()
+
+    def feed(v):
+        if isinstance(v, (bytes, bytearray)):
+            h.update(b"b%d:" % len(v) + bytes(v))
+        elif isinstance(v, np.ndarray):
+            v = np.ascontiguousarray(v)
+            h.update(("a%s%s:" % (v.dtype.str, v.shape)).encode() + v.tobytes())
+        elif isinstance(v, str):
+            h.update(b"t%d:" % len(v) + v.encode())
+        elif isinstance(v, C.Structure):
+            h.update(b"s:" + bytes(v))
+        elif isinstance(v, (bool, int, np.integer)):
+            h.update(b"i%d;" % int(v))
+        elif isinstance(v, (tuple, list)):
+            h.update(b"(%d" % len(v))
+            for e in v:
+                feed(e)
+            h.update(b")")
+        elif v is None:
+            h.update(b"n;")
+        else:
+            raise TypeError(type(v))
+    feed(x)
+    return h.hexdigest()
+
+
+class Recorded:
+    """the reference's answer known only by its recorded digest (no reference build on this machine)"""
+
+    def __init__(self, key, sha):
+        self.key, self.sha = key, sha
+
+    def __repr__(self):
+        return "Recorded(%r)" % self.key
+
+
+def same(a, b):
+    """a (the product's result) equals b (from_reference(), a live result or a Recorded digest)"""
+    return digest(a) == (b.sha if isinstance(b, Recorded) else digest(b))
+
+
+def _recorded(key):
+    global _digests_cache
+    if _digests_cache is None:
+        import json
+        _digests_cache = json.load(open(REF_DIGESTS)) if os.path.exists(REF_DIGESTS) else {}
+    sha = _digests_cache.get(key)
+    assert sha is not None, "no recorded reference result for %r in %s" % (key, REF_DIGESTS)
+    return sha
+
+
+def _record(key, value, blob=False):
+    """under UHDR_RECORD_REFERENCE=<dir>: add key -> digest (and the bytes themselves when blob) to <dir>"""
+    d = os.environ.get("UHDR_RECORD_REFERENCE")
+    if not d:
+        return
+    import json
+    os.makedirs(d, exist_ok=True)
+    p = os.path.join(d, "reference_digests.json")
+    cur = json.load(open(p)) if os.path.exists(p) else {}
+    cur[key] = digest(value)
+    with open(p, "w") as f:
+        json.dump(cur, f, indent=0, sort_keys=True)
+        f.write("\n")
+    if blob:
+        os.makedirs(os.path.join(d, "reference"), exist_ok=True)
+        with open(os.path.join(d, "reference", _blob_name(key)), "wb") as f:
+            f.write(value)
+
+
+def _blob_name(key):
+    import re
+    return re.sub(r"[^A-Za-z0-9_.-]+", "_", key).strip("_") + ".bin"
+
+
+def from_reference(key, fn):
+    """the reference's answer for `key`: fn() when the reference build is present, else its recorded digest"""
+    if have_ref():
+        v = fn()
+        _record(key, v)
+        return v
+    return Recorded(key, _recorded(key))
+
+
+def reference_file(key, fn, mine=None):
+    """bytes (or a tuple of results) the reference produced, needed as an INPUT by a test: fn() when the
+    reference build is present, and then mine() -- the product's or the C restatement's way of making
+    them -- must return the same.  Otherwise mine() must reproduce the recorded digest exactly; without
+    mine, the bytes stored under tests/golden/reference/ are used (and checked against the digest)."""
+    if have_ref():
+        v = fn()
+        _record(key, v, blob=mine is None)
+        if mine is not None:
+            assert same(mine(), v), "%s differs from what the reference produced" % key
+        return v
+    sha = _recorded(key)
+    if mine is not None:
+        v = mine()
+    else:
+        with open(os.path.join(REF_BLOBS, _blob_name(key)), "rb") as f:
+            v = f.read()
+    assert digest(v) == sha, "%s differs from what the reference produced" % key
+    return v
 
 
 # ------------------------------------------------------------------------------------------------
@@ -121,9 +243,13 @@ def make_rgba8888(w, h, seed=SEED + 4):
 
 
 def load_fixture_720p():
-    """config 1 inputs; only available in the build container (not on the GPU box)."""
-    p = np.fromfile(os.path.join(REF_DATA, "raw_p010_image.p010"), dtype=np.uint16)
-    y = np.fromfile(os.path.join(REF_DATA, "raw_yuv420_image.yuv420"), dtype=np.uint8)
+    """config 1 inputs: the reference's 1280x720 colour-bar fixtures (tests/data/raw_p010_image.p010 and
+    raw_yuv420_image.yuv420 of libultrahdr), stored xz-compressed under tests/golden/."""
+    import lzma
+    with lzma.open(os.path.join(GOLDEN, "raw_p010_image.p010.xz")) as f:
+        p = np.frombuffer(f.read(), dtype=np.uint16).copy()
+    with lzma.open(os.path.join(GOLDEN, "raw_yuv420_image.yuv420.xz")) as f:
+        y = np.frombuffer(f.read(), dtype=np.uint8).copy()
     return p, y
 
 
