@@ -25,6 +25,9 @@ struct uhdr_codec_private {
   int init_rc = 0;
   int device = -1;  // the CUDA device that was current when the handle was created
   std::string init_err;
+  // uhdr_add_effect_* in call order; cleared by reset, keeping its capacity.  Planned into one gather per image
+  // (effects.h) when the handle sails.
+  std::vector<Effect> effects;
   uhdr_codec_private() {
     if (cudaGetDevice(&device) != cudaSuccess) device = -1;
   }
@@ -92,6 +95,7 @@ struct Encoder : uhdr_codec_private {
     scale = 1; multichannel = 1; preset = UHDR_USAGE_BEST_QUALITY; output_format = UHDR_CODEC_JPG;
     gamma = 1.0f; min_boost = FLT_MIN; max_boost = FLT_MAX; target_nits = -1.0f;
     has_compressed = false;
+    effects.clear();
     sailed = false;
     memset(&out_desc, 0, sizeof out_desc);
     status = ok();
@@ -112,6 +116,7 @@ struct Decoder : uhdr_codec_private {
   uhdr_error_info_t probe_status = ok(), status = ok();
   void defaults() {
     stream.clear();
+    effects.clear();
     out_fmt = UHDR_IMG_FMT_64bppRGBAHalfFloat;
     out_ct = UHDR_CT_LINEAR;
     max_boost = FLT_MAX;
@@ -348,7 +353,21 @@ UHDR_API uhdr_error_info_t uhdr_encode(uhdr_codec_private_t* enc) {
     h->status = err(UHDR_CODEC_INVALID_OPERATION, "resources required for uhdr_encode() operation are not present");
     return h->status;
   }
+  // image effects (:1219-1262): raw intents only, planned and validated before the device is touched
+  const bool fx = !h->effects.empty();
+  ImageMap fx_hdr{}, fx_sdr{};
+  if (fx) {
+    if (api4 || csdr != h->compressed.end()) {
+      h->status = err(UHDR_CODEC_INVALID_OPERATION, "image effects are not enabled for inputs with compressed intent");
+      return h->status;
+    }
+    const int rc = plan_encoder_effects(h->effects.data(), (int)h->effects.size(), hdr->second.v.fmt,
+                                        sdr == h->raw.end() ? -1 : sdr->second.v.fmt, hdr->second.v.w, hdr->second.v.h,
+                                        &fx_hdr, &fx_sdr);
+    if (rc) { h->status = from_rc(rc); return h->status; }
+  }
   const size_t cap = api4 ? std::max<size_t>(64 * 1024, 2 * (cbase->second.bytes.size() + cgm->second.bytes.size()))
+                   : fx   ? std::max<size_t>(64 * 1024, (size_t)fx_hdr.w * fx_hdr.h * 3 * 2)
                           : std::max<size_t>(64 * 1024, (size_t)hdr->second.v.w * hdr->second.v.h * 3 * 2);  // :1281,:1294
   if (h->out_cap < cap) {
     h->out.reset(new (std::nothrow) uint8_t[cap]);
@@ -378,9 +397,18 @@ UHDR_API uhdr_error_info_t uhdr_encode(uhdr_codec_private_t* enc) {
     if (csdr != h->compressed.end())  // API-2 (raw sdr intent given too) / API-3
       rc = h->codec.encode_with_compressed_sdr(hdr->second, sdr == h->raw.end() ? nullptr : &sdr->second, csdr->second.bytes.data(),
                                                csdr->second.bytes.size(), csdr->second.cg, cfg, h->out.get(), cap, &n);
-    else
-      rc = h->codec.encode(hdr->second, sdr == h->raw.end() ? nullptr : &sdr->second, cfg, h->quality[UHDR_BASE_IMG],
-                           h->exif.empty() ? nullptr : h->exif.data(), h->exif.size(), h->out.get(), cap, &n);
+    else {
+      // the effects gather the resident intents into per-encode scratch above the arena floor: the inputs are
+      // never written, so a re-armed handle encodes the same bytes again
+      DevImage hdr_img = hdr->second, sdr_img;
+      if (sdr != h->raw.end()) sdr_img = sdr->second;
+      rc = E_OK;
+      if (fx) rc = apply_effects_dev(h->codec.ws(), hdr->second, fx_hdr, &hdr_img);
+      if (fx && rc == E_OK && sdr != h->raw.end()) rc = apply_effects_dev(h->codec.ws(), sdr->second, fx_sdr, &sdr_img);
+      if (rc == E_OK)
+        rc = h->codec.encode(hdr_img, sdr == h->raw.end() ? nullptr : &sdr_img, cfg, h->quality[UHDR_BASE_IMG],
+                             h->exif.empty() ? nullptr : h->exif.data(), h->exif.size(), h->out.get(), cap, &n);
+    }
   }
   h->status = from_rc(rc);
   if (rc == E_OK) {
@@ -501,6 +529,14 @@ UHDR_API uhdr_error_info_t uhdr_decode(uhdr_codec_private_t* dec) {
     h->status = err(UHDR_CODEC_INVALID_PARAM, "unsupported output pixel format and output color transfer pair");
     return h->status;
   }
+  // image effects (:1996-1998, :289-429): planned from the probed sizes, so every error comes before device work
+  const bool fx = !h->effects.empty();
+  ImageMap fx_img{}, fx_map{};
+  if (fx) {
+    const int rc = plan_decoder_effects(h->effects.data(), (int)h->effects.size(), h->info.width, h->info.height,
+                                        h->info.gm_width, h->info.gm_height, &fx_img, &fx_map);
+    if (rc) { h->status = from_rc(rc); return h->status; }
+  }
   h->ensure();
   if (h->init_rc) { h->status = err((uhdr_codec_err_t)h->init_rc, "%s", h->init_err.c_str()); return h->status; }
   const int w = h->info.width, ht = h->info.height;
@@ -522,7 +558,8 @@ UHDR_API uhdr_error_info_t uhdr_decode(uhdr_codec_private_t* dec) {
   h->gainmap_desc.stride[0] = h->info.gm_width;
   h->codec.set_lazy_gainmap(true);  // the map leaves HBM only if uhdr_get_decoded_gainmap_image() is called
   int rc = h->codec.decode(h->stream.data(), h->stream.size(), h->out_ct, h->out_fmt, h->max_boost, &h->decoded_desc,
-                           &h->gainmap_desc, nullptr, &h->info);   // uhdr_dec_probe above already located the two images
+                           &h->gainmap_desc, nullptr, &h->info,   // uhdr_dec_probe above already located the two images
+                           fx ? &fx_img : nullptr, fx ? &fx_map : nullptr);
   h->status = from_rc(rc);
   return h->status;
 }
@@ -550,14 +587,36 @@ UHDR_API uhdr_error_info_t uhdr_enable_gpu_acceleration(uhdr_codec_private_t* co
   if (!codec) return err(UHDR_CODEC_INVALID_PARAM, "received nullptr for uhdr codec instance");
   return ok();  // the CUDA path is the only path
 }
-static uhdr_error_info_t no_effects(uhdr_codec_private_t* codec) {
+// uhdr_add_effect_*, ultrahdr_api.cpp:2113-2229: arguments are checked here, sizes when the handle sails
+#define EFFECT_NULL_CHECK \
   if (!codec) return err(UHDR_CODEC_INVALID_PARAM, "received nullptr for uhdr codec instance");
-  return err(UHDR_CODEC_UNSUPPORTED_FEATURE, "image effects (editorhelper.cpp) are outside the B200 hot path");
+static uhdr_error_info_t add_effect(uhdr_codec_private_t* codec, const Effect& e) {
+  if (codec->sailed)
+    return err(UHDR_CODEC_INVALID_OPERATION, "An earlier call to uhdr_encode()/uhdr_decode() has switched the context "
+               "from configurable state to end state. The context is no longer configurable. To reuse, call reset()");
+  codec->effects.push_back(e);
+  return ok();
 }
-UHDR_API uhdr_error_info_t uhdr_add_effect_mirror(uhdr_codec_private_t* c, uhdr_mirror_direction_t) { return no_effects(c); }
-UHDR_API uhdr_error_info_t uhdr_add_effect_rotate(uhdr_codec_private_t* c, int) { return no_effects(c); }
-UHDR_API uhdr_error_info_t uhdr_add_effect_crop(uhdr_codec_private_t* c, int, int, int, int) { return no_effects(c); }
-UHDR_API uhdr_error_info_t uhdr_add_effect_resize(uhdr_codec_private_t* c, int, int) { return no_effects(c); }
+UHDR_API uhdr_error_info_t uhdr_add_effect_mirror(uhdr_codec_private_t* codec, uhdr_mirror_direction_t direction) {
+  EFFECT_NULL_CHECK
+  if (direction != UHDR_MIRROR_HORIZONTAL && direction != UHDR_MIRROR_VERTICAL)
+    return err(UHDR_CODEC_INVALID_PARAM, "unsupported direction, expects one of {UHDR_MIRROR_HORIZONTAL, UHDR_MIRROR_VERTICAL}");
+  return add_effect(codec, Effect{FX_MIRROR, (int)direction, 0, 0, 0});
+}
+UHDR_API uhdr_error_info_t uhdr_add_effect_rotate(uhdr_codec_private_t* codec, int degrees) {
+  EFFECT_NULL_CHECK
+  if (degrees != 90 && degrees != 180 && degrees != 270)
+    return err(UHDR_CODEC_INVALID_PARAM, "unsupported degrees, expects one of {90, 180, 270}");
+  return add_effect(codec, Effect{FX_ROTATE, degrees, 0, 0, 0});
+}
+UHDR_API uhdr_error_info_t uhdr_add_effect_crop(uhdr_codec_private_t* codec, int left, int right, int top, int bottom) {
+  EFFECT_NULL_CHECK
+  return add_effect(codec, Effect{FX_CROP, left, right, top, bottom});
+}
+UHDR_API uhdr_error_info_t uhdr_add_effect_resize(uhdr_codec_private_t* codec, int width, int height) {
+  EFFECT_NULL_CHECK
+  return add_effect(codec, Effect{FX_RESIZE, width, height, 0, 0});
+}
 
 // ---- measurement hooks (include/uhdr_b200.h) -------------------------------------------------------
 UHDR_API void uhdr_b200_set_kernel_timing(int on) { set_kernel_timing(on != 0); }

@@ -413,7 +413,7 @@ int JpegRCodec::probe(const uint8_t* data, size_t size, DecodedInfo* info) {
 
 int JpegRCodec::decode(const uint8_t* data, size_t size, int out_ct, int out_fmt, float max_display_boost,
                        uhdr_raw_image_t* dest, uhdr_raw_image_t* gainmap_out, uhdr_gainmap_metadata_t* md_out,
-                       const DecodedInfo* probed) {
+                       const DecodedInfo* probed, const ImageMap* fx_img, const ImageMap* fx_map) {
   (void)out_fmt;
   PhaseTrace tr;
   ws_.rewind();
@@ -492,23 +492,29 @@ int JpegRCodec::decode(const uint8_t* data, size_t size, int out_ct, int out_fmt
     if (md_out) *md_out = md;
   }
   if (gainmap_out) {
-    gainmap_out->fmt = (uhdr_img_fmt_t)map.v.fmt;
-    gainmap_out->w = map.v.w;
-    gainmap_out->h = map.v.h;
+    DevImage gm = map;  // `map` itself stays as decoded: the gain map is applied untransformed
+    if (fx_map) {
+      rc = apply_effects_dev(ws_, map, *fx_map, &gm);
+      if (rc) return rc;
+    }
+    const int gm_stride = fx_map ? gm.v.stride[0] : gm.v.w;
+    gainmap_out->fmt = (uhdr_img_fmt_t)gm.v.fmt;
+    gainmap_out->w = gm.v.w;
+    gainmap_out->h = gm.v.h;
     gainmap_out->cg = UHDR_CG_UNSPECIFIED;
     gainmap_out->ct = UHDR_CT_UNSPECIFIED;
     gainmap_out->range = UHDR_CR_FULL_RANGE;
     if (!gainmap_out->planes[0] && lazy_gainmap_) {
-      gainmap_out->stride[0] = map.v.w;
-      last_map_ = map;
+      gainmap_out->stride[0] = gm_stride;
+      last_map_ = gm;
       map_pending_ = true;
     } else {
       if (!gainmap_out->planes[0]) {  // handle-owned result: pinned memory of this codec, valid until its next decode
-        gainmap_out->stride[0] = map.v.w;
-        gainmap_out->planes[0] = ws_.halloc((size_t)map.v.w * map.v.h * (map.v.fmt == F_Y400 ? 1 : 4));
+        gainmap_out->stride[0] = gm_stride;
+        gainmap_out->planes[0] = ws_.halloc((size_t)gm_stride * gm.v.h * (gm.v.fmt == F_Y400 ? 1 : 4));
         if (!gainmap_out->planes[0]) return E_MEM;
       }
-      rc = download_image(ws_, map, gainmap_out);
+      rc = download_image(ws_, gm, gainmap_out);
       if (rc) return rc;
     }
   }
@@ -528,14 +534,36 @@ int JpegRCodec::decode(const uint8_t* data, size_t size, int out_ct, int out_fmt
     dest->ct = (uhdr_color_transfer_t)out_ct;
   }
   dest->range = UHDR_CR_FULL_RANGE;
-  if (!dest->planes[0]) {  // handle-owned result (see above)
-    dest->stride[0] = sdr.v.w;
-    dest->planes[0] = ws_.halloc((size_t)sdr.v.w * sdr.v.h * (dest->fmt == UHDR_IMG_FMT_64bppRGBAHalfFloat ? 8 : 4));
-    if (!dest->planes[0]) return E_MEM;
+  const size_t bpp = dest->fmt == UHDR_IMG_FMT_64bppRGBAHalfFloat ? 8 : 4;
+  if (fx_img) {
+    // the effects run on the device image, and only their result crosses to the host; the gather wrote
+    // whole rows up to the stride (zeros past the width), so they go as one linear copy
+    DevImage fx;
+    rc = apply_effects_dev(ws_, dst, *fx_img, &fx);
+    if (rc) return rc;
+    const size_t bytes = (size_t)fx.v.stride[0] * fx.v.h * bpp;
+    dest->w = fx.v.w;
+    dest->h = fx.v.h;
+    if (!dest->planes[0]) {
+      dest->stride[0] = fx.v.stride[0];
+      dest->planes[0] = ws_.halloc(bytes);
+      if (!dest->planes[0]) return E_MEM;
+    }
+    tr.mark("apply + effects enqueued");
+    if ((int)dest->stride[0] == fx.v.stride[0])
+      CUDA_TRY(cudaMemcpyAsync(dest->planes[0], fx.v.p[0], bytes, cudaMemcpyDeviceToHost, ws_.stream()));
+    else if ((rc = download_image(ws_, fx, dest)))
+      return rc;
+  } else {
+    if (!dest->planes[0]) {  // handle-owned result (see above)
+      dest->stride[0] = sdr.v.w;
+      dest->planes[0] = ws_.halloc((size_t)sdr.v.w * sdr.v.h * bpp);
+      if (!dest->planes[0]) return E_MEM;
+    }
+    tr.mark("apply enqueued");
+    rc = download_image(ws_, dst, dest);
+    if (rc) return rc;
   }
-  tr.mark("apply enqueued");
-  rc = download_image(ws_, dst, dest);
-  if (rc) return rc;
   rc = ws_.sync();
   tr.mark("pixels on the host");
   return rc;
@@ -543,7 +571,7 @@ int JpegRCodec::decode(const uint8_t* data, size_t size, int out_ct, int out_fmt
 
 int JpegRCodec::fetch_gainmap(uhdr_raw_image_t* gainmap_out) {
   if (!map_pending_) return E_OK;
-  gainmap_out->planes[0] = ws_.halloc((size_t)last_map_.v.w * last_map_.v.h * (last_map_.v.fmt == F_Y400 ? 1 : 4));
+  gainmap_out->planes[0] = ws_.halloc((size_t)gainmap_out->stride[0] * last_map_.v.h * (last_map_.v.fmt == F_Y400 ? 1 : 4));
   if (!gainmap_out->planes[0]) return E_MEM;
   int rc = download_image(ws_, last_map_, gainmap_out);
   if (rc) return rc;

@@ -9,6 +9,7 @@
 #include <vector>
 
 #include "container.h"
+#include "effects.h"
 #include "engine.h"
 #include "jpeg.h"
 
@@ -67,9 +68,11 @@ class JpegRCodec {
   // JpegR::decodeJPEGR (jpegr.cpp:1469-1531).  dest: host descriptor with planes allocated by the
   // caller (fmt/stride set); gainmap_out optional host descriptor (planes allocated, Y400/RGBA8888).
   // `probed`: the result of probe() on the same stream (saves the second scan of the container), or null.
+  // `fx_img` / `fx_map`: image effects planned for the decoded image and the gain map (plan_decoder_effects),
+  // or null.  With effects the descriptors report the transformed size at stride ALIGNM(w, 64).
   int decode(const uint8_t* data, size_t size, int out_ct, int out_fmt, float max_display_boost,
              uhdr_raw_image_t* dest, uhdr_raw_image_t* gainmap_out, uhdr_gainmap_metadata_t* md_out,
-             const DecodedInfo* probed = nullptr);
+             const DecodedInfo* probed = nullptr, const ImageMap* fx_img = nullptr, const ImageMap* fx_map = nullptr);
 
   // With gainmap_out->planes[0] == nullptr and lazy_gainmap set, decode() only fills the descriptor's
   // geometry and keeps the map in HBM; fetch_gainmap() copies it out when somebody asks for it
